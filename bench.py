@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # ours (sm_100a kernels)
   python bench.py --impl reference --steps K --warmup W    # reference-equivalent CPU path (oracle port)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 Headline workload (BASELINE.json configs[1]): dagr-s, events only, synthetic DSEC-shaped 640x480 streams,
 50 ms window, 300k events/sample, batch 8 per GPU.  A "step" is one synchronous forward
@@ -52,7 +53,14 @@ def parse():
     p.add_argument("--sustained-seconds", type=float, default=2.0)
     p.add_argument("--headline-only", action="store_true", help="skip clustered / sustained / config 3 / config 5 / config 4")
     p.add_argument("--stream-seconds", type=float, default=2.0, help="length of the config-5 stream")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the headline loop returned (decoded "
+                                                         "outputs, detections) as DIR/<name>.npy, to compare two builds")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be >= 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs applies to the GPU arm (--impl ours)")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------
@@ -164,6 +172,16 @@ def margs_size(a):
 def _pct(xs, q):
     xs = sorted(xs)
     return xs[min(len(xs) - 1, int(q * len(xs)))]
+
+
+def host_outputs(dec, det, ndet):
+    """one step's results on the host: decoded [B, anchors, 5 + classes] (forward_decoded), detections [B, anchors, 6]
+    (x1, y1, x2, y2, score, label; the NMS kernel leaves the rows past num_detections unwritten, they are stored as 0) and
+    num_detections [B]."""
+    det, ndet = det.float().cpu(), ndet.cpu()
+    for b in range(len(ndet)):
+        det[b, int(ndet[b]):] = 0
+    return dict(decoded=dec.float().cpu().numpy(), detections=det.numpy(), num_detections=ndet.double().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -313,11 +331,12 @@ def main():
                 with mdl.engine.result_stream():
                     det, ndet = parallel.all_gather_detections(det, ndet)
                 mdl.engine.fence()
-            return det, ndet
+            return dec, det, ndet
         return mdl, raws_, dev_in_, nev, step_
 
     def timed(eng_, step_, nsteps, warm):
-        """W warm-up steps, then exactly `nsteps` steps between barriers; CUDA events; max over ranks."""
+        """W warm-up steps, then exactly `nsteps` steps between barriers; CUDA events; max over ranks.
+        -> (ms per step, launches, what the last step returned)"""
         for i in range(warm):
             step_(i)
         barrier()
@@ -326,11 +345,11 @@ def main():
         barrier()
         e0.record()
         for i in range(nsteps):
-            step_(i)
+            out = step_(i)
         eng_.join()                                              # the last steps' side-stream work is inside the timed region
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1) / nsteps), eng_.launches - l0
+        return max_over_ranks(e0.elapsed_time(e1) / nsteps), eng_.launches - l0, out
 
     model, raws, dev_in, n_events, step = make_workload(a.size, a.kind, 42 + 1000 * 2)
     eng = model.engine
@@ -347,23 +366,24 @@ def main():
         step(i)
     barrier()
     c0 = sampler.mark()
-    ms, launches = timed(eng, step, a.steps, 0)
+    ms, launches, last = timed(eng, step, a.steps, 0)
     c1 = sampler.mark()
     value = n_events * world / (ms * 1e-3) / 1e6
+    dumped = host_outputs(*last) if a.dump_outputs and rank == 0 else None   # copied now: later runs reuse the buffers
 
     # ---- sustained: >= 2 s of back-to-back steps (same loop, same inputs) with clock samples ----------
     sustained = None
     if not a.headline_only:
         n_sus = max(a.steps, int(a.sustained_seconds / (ms * 1e-3)) + 1)
         s0 = sampler.mark()
-        sms, _ = timed(eng, step, n_sus, 0)
+        sms, _, _ = timed(eng, step, n_sus, 0)
         s1 = sampler.mark()
         sustained = dict(value=n_events * world / (sms * 1e-3) / 1e6, unit=UNIT, steps=n_sus, ms_per_step=sms, seconds=sms * n_sus * 1e-3,
                          clocks=sampler.summary(s0, s1))
 
     # ---- latency of ONE forward (serial: no overlap between consecutive steps) --------------------
     eng.overlap = False
-    serial_ms, _ = timed(eng, step, a.steps, 3)
+    serial_ms, _, _ = timed(eng, step, a.steps, 3)
 
     # ---- e2e through the public API from pinned host memory --------------------------------------
     from dagr_b200.pipeline import PipelinedDetector, Prefetcher
@@ -489,7 +509,7 @@ def main():
         del dev_in
         m2, _, _, nev2, step2 = make_workload(a.size, other, 42 + 1000 * 2)
         m2.engine.overlap = not a.no_overlap
-        ms2, _ = timed(m2.engine, step2, a.steps, warm)
+        ms2, _, _ = timed(m2.engine, step2, a.steps, warm)
         m2.engine.overlap = False
         prof2, N2, E2 = per_op(m2, step2, min(a.steps, 10))
         line[other] = dict(value=nev2 * world / (ms2 * 1e-3) / 1e6, unit=UNIT, ms_per_step=ms2, mean_degree=E2 / max(N2, 1),
@@ -501,7 +521,7 @@ def main():
         if world > 1:
             m4, _, _, nev4, step4 = make_workload("m", a.kind, 42 + 1000 * 4)
             m4.engine.overlap = not a.no_overlap
-            ms4, _ = timed(m4.engine, step4, a.steps, warm)
+            ms4, _, _ = timed(m4.engine, step4, a.steps, warm)
             line.setdefault("extra", {})["config4"] = dict(model="dagr-m", global_batch=a.batch * world, value=nev4 * world / (ms4 * 1e-3) / 1e6,
                                                            unit=UNIT, ms_per_step=ms4, n_gpus=world)
             del m4, step4
@@ -537,6 +557,12 @@ def main():
         n_target = int(min(a.events, max(2000, cal["events"] * (a.cpu_seconds / 2) / max(cal["sec_per_step"], 1e-3))))
         r = cpu_reference_run(sd, margs, raws[0], n_target, 2, 0, threads)
         line["cpu_baseline"] = dict(value=r["mev_s"], unit=UNIT, cores=threads, kind="port", sample=r["sample"])
+    if dumped is not None:
+        import numpy as np
+        out = Path(a.dump_outputs)
+        out.mkdir(parents=True, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(out / f"{name}.npy", arr)
     if rank == 0:
         print(json.dumps(line))
     if world > 1:

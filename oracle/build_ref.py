@@ -6,10 +6,9 @@ under /root/reference (nothing is copied into this repo) into oracle/_ref/:
   ev_graph_cuda  <- /root/reference/src/dagr/graph/ev_graph.cu (+ spiral.h)       (setup.py:8-9)
   asy_tools      <- /root/reference/src/dagr/asynchronous/asy_tools/main.cu      (setup.py:10-11)
 
-The products are git-ignored (oracle/_ref/) but travel to the GPU box with the gpurun
-snapshot, where the `-m gpu` tests load them to check our kernels against the real
-reference kernels on identical inputs.  /root/reference does not exist on the GPU box;
-there this script is a no-op when the prebuilt .so files are present.
+The products are git-ignored (oracle/_ref/).  tests/golden/make_reference_kernels_golden.py
+runs them on a GPU to write the fixtures the `-m gpu` tests compare our kernels against.
+Without the reference sources this script builds nothing.
 """
 import os
 import sys

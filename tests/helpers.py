@@ -148,6 +148,38 @@ def load_reference_fixture(name):
     return model, args, data, exp, dict(W=W, H=H, B=B, use_image=bool(use_image), num_scales=nscale)
 
 
+def sha256(*tensors) -> str:
+    """hex SHA-256 of the tensors' bytes (C order, dtype as given): pins inputs and outputs too large to store."""
+    import hashlib
+    h = hashlib.sha256()
+    for t in tensors:
+        h.update(np.ascontiguousarray(t.detach().cpu().numpy()).tobytes())
+    return h.hexdigest()
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# inputs of the comparisons with the reference's own CUDA extensions (fixtures: tests/golden/make_reference_kernels_golden.py)
+# ------------------------------------------------------------------------------------------------------------------
+# dagr-n, make_inputs(B, n, W, H, seed, kind); K = max_neighbors, Q = max_queue_size of the reference's graph builder
+REF_GRAPH_CASE = dict(W=320, H=215, B=2, n=40000, seed=21, kind="clustered", K=16, Q=128)
+
+
+def masked_ops_inputs(dev):
+    """seeded inputs of the masked linear / batch-norm / is-different kernels of the asynchronous path."""
+    g = torch.Generator().manual_seed(0)
+    Rn, Cin, Cout, K = 500, 18, 64, 77
+    t = dict(idx=torch.randperm(Rn, generator=g)[:K], x=torch.randn(Rn, Cin, generator=g), w=torch.randn(Cout, Cin, generator=g),
+             b=torch.randn(Cout, generator=g), base=torch.randn(Rn, Cout, generator=g), mean=torch.randn(Cout, generator=g),
+             var=torch.rand(Cout, generator=g) + 0.5, gamma=torch.rand(Cout, generator=g) + 0.5, beta=torch.randn(Cout, generator=g),
+             xin=torch.randn(Rn, Cout, generator=g), a=torch.rand(Rn, Cin, generator=g) + 0.5)
+    idx, a = t["idx"], t["a"]
+    c = a.clone()
+    c[idx[::3], 3] += 0.5
+    a[idx[1], 0] = -2.0; c[idx[1], 0] = -2.0                         # quirk Q3 row
+    t["c"] = c
+    return {k: v.to(dev) for k, v in t.items()}
+
+
 def image_branch_cpu(model, data):
     """the dense image trunk + CNN head on the CPU in fp32 (library code on both sides): the tensors the graph path consumes."""
     with torch.no_grad():

@@ -1,32 +1,20 @@
-"""GPU parity suite: hand-written sm_100a kernels (through the C-ABI) against the CPU oracle, and --
-where the reference's own CUDA extensions were compiled into oracle/_ref -- against the reference
-kernels themselves.  Integer results bit-exact; fp32 features within 1e-4 relative (tests/helpers.py).
+"""GPU parity suite: hand-written sm_100a kernels (through the C-ABI) against the CPU oracle, and against the
+outputs of the reference's own CUDA kernels stored under tests/golden.  Integer results bit-exact; fp32 features
+within 1e-4 relative (tests/helpers.py).
 """
-import sys
 from pathlib import Path
 
 import numpy as np
 import pytest
 import torch
 
-from tests.helpers import REFERENCE_FIXTURES, RTOL, assert_close, make_inputs, make_model, rel_err
+from tests.helpers import (REF_GRAPH_CASE, REFERENCE_FIXTURES, RTOL, assert_close, make_inputs, make_model, masked_ops_inputs,
+                           rel_err, sha256)
 
 pytestmark = pytest.mark.gpu
 ROOT = Path(__file__).resolve().parent.parent
+GOLD = ROOT / "tests" / "golden"
 DUMP = ROOT / "gpurun_out"
-
-
-def _ref_ext(name):
-    d = ROOT / "oracle" / "_ref" / name
-    if not any(d.glob(f"{name}*.so")):
-        return None
-    if str(d) not in sys.path:
-        sys.path.insert(0, str(d))
-    try:
-        return __import__(name)
-    except Exception as e:                      # pragma: no cover
-        print(f"could not import reference extension {name}: {e}")
-        return None
 
 
 def _run_graph(model, data, B):
@@ -174,34 +162,30 @@ def test_graph_empty_and_single_event():
         assert len(out[0]) == 1
 
 
+def _assert_reference_graph_edges(e, gold, who):
+    """edge_index int64[2, E] == the reference kernels' (tests/golden/reference_graph_kernels.npz): every edge of the
+    stored sample of destination events, then the edge count and the SHA-256 of the whole edge_index."""
+    e = e.cpu().long()
+    keep = torch.from_numpy(np.isin(e[1].numpy(), gold["sample_dst"]))
+    assert torch.equal(e[:, keep], torch.from_numpy(gold["sample_edges"]).long()), f"{who}: edges of the sampled events"
+    assert e.shape[1] == int(gold["num_edges"]), (who, e.shape[1], int(gold["num_edges"]))
+    assert sha256(e) == str(gold["edges_sha256"]), f"{who}: edge_index differs from the reference kernels'"
+
+
 def test_graph_vs_reference_cuda_kernels():
-    """our edge_index == the reference's own insert_in_queue_cuda + fill_edges_cuda (oracle/_ref)."""
-    ext = _ref_ext("ev_graph_cuda")
-    if ext is None:
-        pytest.skip("reference extension not built (oracle/_ref/ev_graph_cuda)")
-    W, H, B, K, Q = 320, 215, 2, 16, 128
+    """our edge_index == the reference's own insert_in_queue_cuda + fill_edges_cuda on the same events (fixture made by
+    tests/golden/make_reference_kernels_golden.py)."""
+    gold = np.load(GOLD / "reference_graph_kernels.npz")
+    c = REF_GRAPH_CASE
+    W, H, B = c["W"], c["H"], c["B"]
     model, args = make_model("n", H, W)
     model.cuda()
-    raw, data = make_inputs(B, 40000, W, H, seed=21, kind="clustered")
+    raw, data = make_inputs(B, c["n"], W, H, seed=c["seed"], kind=c["kind"])
     _, batch_i, pos_i = _run_graph(model, data, B)
-    mine = model.engine.export_edges()
-    # drive the reference kernels exactly as graph/utils.py:6-23 + ev_graph.py:63-103 do
-    N = len(batch_i)
-    dev = batch_i.device
-    queue = torch.full((B, Q, H, W), -1, dtype=torch.int32, device=dev)
-    indices = torch.arange(N, dtype=torch.int32, device=dev)
-    lin = pos_i[:, 0] + W * pos_i[:, 1] + W * H * batch_i
-    s_lin, s_idx = torch.sort(lin, stable=True)
-    uniq, cnt = torch.unique_consecutive(s_lin, return_counts=True)
-    queue = ext.insert_in_queue_cuda(indices[s_idx].int().contiguous(), uniq.contiguous(), torch.cumsum(cnt, 0).int().contiguous(), queue)
-    edges = torch.full((2, K * N), -1, dtype=torch.int64, device=dev)
-    r = int(args.radius * W + 1)
-    ext.fill_edges_cuda(batch_i, pos_i, pos_i[:, 2].contiguous(), queue, indices, K, float(r), float(int(args.radius * 1e6)), edges, 0)
-    torch.cuda.synchronize()
-    ref = edges[:, edges[1] >= 0]
-    assert torch.equal(mine, ref)
+    assert sha256(batch_i.int(), pos_i.int()) == str(gold["inputs_sha256"]), "events differ from the ones the fixture was made from"
+    _assert_reference_graph_edges(model.engine.export_edges(), gold, "CUDA path")
     # and the C oracle agrees with the reference kernels too (pins oracle/graph_oracle.c)
-    assert torch.equal(_oracle_graph(args, W, H, B, batch_i, pos_i), ref.cpu())
+    _assert_reference_graph_edges(_oracle_graph(args, W, H, B, batch_i, pos_i), gold, "C oracle")
 
 
 # ---------------------------------------------------------------------------------------------
@@ -622,13 +606,18 @@ def test_masked_ops_vs_oracle_and_reference():
     from dagr_b200 import _lib
     from oracle import ref_ops as R
     lib = _lib.load()
-    torch.manual_seed(0)
-    Rn, Cin, Cout, K = 500, 18, 64, 77
-    dev = "cuda"
-    idx = torch.randperm(Rn)[:K].to(dev)
-    x = torch.randn(Rn, Cin, device=dev); w = torch.randn(Cout, Cin, device=dev); b = torch.randn(Cout, device=dev)
-    base = torch.randn(Rn, Cout, device=dev)
-    ext = _ref_ext("asy_tools")
+    t = masked_ops_inputs("cuda")
+    idx, x, w, b, base = t["idx"], t["x"], t["w"], t["b"], t["base"]
+    K, Cin, Cout = len(idx), x.shape[1], w.shape[0]
+    # outputs of the reference's own asy_tools kernels on these inputs (tests/golden/make_reference_kernels_golden.py)
+    gold = np.load(GOLD / "reference_masked_ops.npz")
+    assert sha256(*(t[k] for k in sorted(t))) == str(gold["inputs_sha256"]), "inputs differ from the ones the fixture was made from"
+
+    def reference(name):
+        o = base.cpu().clone()
+        o[idx.cpu()] = torch.from_numpy(gold[name])                   # the reference kernels write the indexed rows only
+        return o
+
     for add in (0, 1):
         for bias in (b, None):
             out = base.clone()
@@ -636,38 +625,22 @@ def test_masked_ops_vs_oracle_and_reference():
                                            _lib.stream_ptr()))
             ref = R.masked_lin(idx.cpu(), x.cpu(), base.cpu().clone(), w.cpu(), None if bias is None else bias.cpu(), bool(add))
             assert_close(out.cpu(), ref, tol=1e-5, what="masked_lin")
-            if ext is not None:
-                o2 = base.clone()
-                if bias is None:
-                    ext.masked_lin_no_bias(idx, x, o2, w, bool(add))
-                else:
-                    ext.masked_lin(idx, x, o2, w, bias, bool(add))
-                assert_close(out.cpu(), o2.cpu(), tol=1e-6, what="masked_lin vs reference asy_tools")
-    mean = torch.randn(Cout, device=dev); var = torch.rand(Cout, device=dev) + 0.5
-    g = torch.rand(Cout, device=dev) + 0.5; be = torch.randn(Cout, device=dev)
-    xin = torch.randn(Rn, Cout, device=dev)
+            o2 = reference(f"masked_lin_add{add}" if bias is not None else f"masked_lin_no_bias_add{add}")
+            assert_close(out.cpu(), o2, tol=1e-6, what="masked_lin vs reference asy_tools")
+    mean, var, g, be, xin = t["mean"], t["var"], t["gamma"], t["beta"], t["xin"]
     out = base.clone()
     _lib.check(lib.dagr_masked_inplace_bn(_lib.ptr(idx), K, _lib.ptr(xin), _lib.ptr(out), _lib.ptr(mean), _lib.ptr(var), _lib.ptr(g),
                                           _lib.ptr(be), Cout, 1e-5, _lib.stream_ptr()))
     ref = R.masked_inplace_bn(idx.cpu(), xin.cpu(), base.cpu().clone(), mean.cpu(), var.cpu(), g.cpu(), be.cpu(), 1e-5)
     assert_close(out.cpu(), ref, tol=1e-5, what="masked_inplace_bn")
-    if ext is not None:
-        o2 = base.clone()
-        ext.masked_inplace_BN(idx, xin, o2, mean, var, g, be, 1e-5)
-        assert_close(out.cpu(), o2.cpu(), tol=1e-6, what="masked_inplace_bn vs reference")
-    a = torch.rand(Rn, Cin, device=dev) + 0.5
-    c = a.clone()
-    changed = idx[::3]
-    c[changed, 3] += 0.5
-    a[idx[1], 0] = -2.0; c[idx[1], 0] = -2.0                         # quirk Q3 row
+    assert_close(out.cpu(), reference("masked_inplace_bn"), tol=1e-6, what="masked_inplace_bn vs reference")
+    a, c = t["a"], t["c"]                                             # c differs from a in column 3 of idx[::3]; Q3 row idx[1]
     cand = idx.clone()
     _lib.check(lib.dagr_masked_isdiff(_lib.ptr(cand), K, _lib.ptr(a), _lib.ptr(c), Cin, 1e-8, 1e-5, _lib.stream_ptr()))
     mine = cand[cand > -1].cpu()
     ref = R.masked_isdiff(idx.cpu(), a.cpu(), c.cpu(), 1e-8, 1e-5)
     assert torch.equal(mine, ref)
-    if ext is not None:
-        r2 = ext.masked_isdiff(idx.clone(), a, c, 1e-8, 1e-5)
-        assert torch.equal(mine, r2.cpu())
+    assert torch.equal(mine, torch.from_numpy(gold["masked_isdiff"]))
 
 
 def test_ingest_downsampler_vs_reference_golden_and_oracle():
